@@ -12,7 +12,8 @@ persistent kernel launch per GPU.  N > 1 shards chains (2048 per GPU, weak scali
 collective).  `value` = leapfrog gradient evaluations (sum of the reference's own `tree_size` stat,
 hmc/nuts.py:485) of all ranks / device time (CUDA events, max over ranks), inputs resident in HBM.
 `e2e` = the same through the public host API with pinned host buffers: H2D of start points / streams
-and D2H of draws + sampler stats inside the timed region.
+and D2H of draws + sampler stats inside the timed region.  `--dump-outputs DIR` writes what the last timed step
+computed as .npy files (the inputs are seeded, so two builds run with the same arguments compare output for output).
 
 The reference arm times oracle/nuts_numpy.py + oracle/logp_numpy.py (the CPU restatement that is
 bit-identical to the reference's own NUTS files; PyTensor is not installable, see DESIGN.md) with one
@@ -87,7 +88,14 @@ def parse():
                     help="logistic / mvgauss: fp64 DMMA (parity mode) or the tcgen05 split-fp16 tensor-core performance mode")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (draws, per-draw stats, per-chain summary) as DIR/<name>.npy "
+                         "in float64; above 64 MB a fixed, seeded sample of chains")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the CUDA engine's outputs: --impl b200")
     args.wl = WORKLOADS[args.workload]
     args.tune = args.wl["tune"] if args.tune < 0 else args.tune
     args.draws = args.wl["draws"] if args.draws < 0 else args.draws
@@ -397,6 +405,31 @@ def make_roofline(workload, wl, per_launch, k_ms, fp64, dmma, peaks, traffic):
 # ---------------------------------------------------------------------------------------------
 # the CUDA engine arm
 # ---------------------------------------------------------------------------------------------
+DUMP_BYTES = 64_000_000  # everything --dump-outputs writes, .npy headers included
+
+
+def dump_outputs(res, out_dir):
+    """Writes the arrays a caller of the timed path receives from one nuts_run -- draws [C, T, n], every per-draw stat
+    [C, T] and every per-chain summary [C, ...] -- as out_dir/<name>.npy in float64, so that two builds run with the same
+    arguments can be compared output for output.  When all chains do not fit in DUMP_BYTES, every array keeps the same
+    chains: a sample drawn from default_rng(0), listed in chains.npy."""
+    import torch
+
+    arrays = {"draws": res.draws, **{"stat_" + k: v for k, v in res.stats.items()},
+              **{"summary_" + k: v for k, v in res.summary.items()}}
+    C = res.draws.shape[0]
+    per_chain = 8 * sum(int(a.numel()) // C for a in arrays.values()) + 8  # float64 values + the chain's index
+    budget = DUMP_BYTES - 4096 * (len(arrays) + 1)  # room for the .npy headers
+    k = min(C, max(1, budget // per_chain))
+    chains = np.arange(C) if k == C else np.sort(np.random.default_rng(0).choice(C, size=k, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "chains.npy"), chains.astype(np.float64))
+    for name, a in arrays.items():
+        sel = a[torch.as_tensor(chains, device=a.device)] if torch.is_tensor(a) else np.asarray(a)[chains]
+        sel = sel.to(torch.float64).cpu().numpy() if torch.is_tensor(sel) else sel.astype(np.float64)
+        np.save(os.path.join(out_dir, name + ".npy"), sel)
+
+
 def pcie_probe(dev, mib=512):
     """Host link of THIS box: one pinned 512 MiB copy each way (CUDA events).  The e2e figure moves with it: the Radon step
     sends 3 GB of draws to the host while the sampling half of the kernel runs."""
@@ -520,6 +553,8 @@ def b200_arm(args):
     evals = parallel.sum_over_ranks(float(evals_t.item()))
     all_evals = float(all_evals_t.item())
     value = evals / (ms_total * 1e-3)
+    if args.dump_outputs and rank == 0:  # rank 0's chains when N > 1
+        dump_outputs(res, args.dump_outputs)
 
     # ESS/sec of the last step (rank-normalised bulk ESS over this rank's chains, min over parameters)
     ess = diagnostics.ess_bulk_torch(res.draws)
@@ -538,7 +573,7 @@ def b200_arm(args):
         mean0_p = None
         if mean0_host is not None:
             mean0_p = pin((C, n), torch.float64); mean0_p[:] = mean0_host
-        n_e2e = max(1, min(args.steps, 3))
+        n_e2e = args.steps
         st_e = states0.copy()
         # one untimed call: allocates the pooled pinned output buffers the timed calls reuse
         res_h = cm.nuts_run(q0_p, st_e, tune=tune, draws=draws, mean0=mean0_p, store_warmup=False,

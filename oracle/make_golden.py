@@ -320,7 +320,176 @@ def full_adapt_cases():
         print(name + "_full_adapt", "grad evals", int(out["stat_tree_size"].sum()), "mean depth", out["stat_depth"].mean())
 
 
+def reference_chain(spec, f, q0, seed, tune, draws, potential, adapt):
+    """One chain of the verbatim reference NUTS from default_rng(seed) -> (positions [T, n], per-draw stats dicts)."""
+    start = {v.name: q0[v.offset : v.offset + v.size].copy() for v in spec.vars}
+    step, _ = ref_loader.make_nuts(f, spec.var_sizes, start, potential=potential, step_rng=0, adapt_step_size=adapt)
+    step.setup_chain(np.random.default_rng(seed), tune, draws)
+    if tune == 0:
+        step.tune = False
+    pt, qs, sts = start, [], []
+    for i in range(tune + draws):
+        if i == tune:
+            step.stop_tuning()
+        pt, st = step.step(pt)
+        qs.append(np.concatenate([np.ravel(pt[v.name]) for v in spec.vars]))
+        sts.append(st[0])
+    return np.array(qs), sts, step
+
+
+def record(out, key, a, limit=2000):
+    """out[key] = a, or -- for an array of more than `limit` values -- its shape and the SHA-256 of its float64 bytes
+    ('<key>.shape', '<key>.sha256'): enough for a bit-identity check at a fraction of the size."""
+    import hashlib
+    a = np.asarray(a)
+    if a.size <= limit:
+        out[key] = a
+    else:
+        out[key + ".shape"] = np.array(a.shape)
+        out[key + ".sha256"] = np.array(hashlib.sha256(np.ascontiguousarray(a, dtype=np.float64).tobytes()).hexdigest())
+
+
+PORT_STAT_KEYS = ["tree_size", "depth", "index_in_trajectory", "energy", "step_size", "step_size_bar", "mean_tree_accept",
+                  "max_energy_error", "model_logp", "diverging", "energy_error"]
+
+
+def port_cases():
+    """ref_port_chains.npz: the reference chains tests/test_oracle_vs_reference.py holds oracle/nuts_numpy.py to, bit for bit
+    (keys '<case>/q' and '<case>/<stat>', large arrays as digests, see record())."""
+    import warnings
+    qp = ref_loader.quadpotential()
+    out = {}
+    for name, adapt, tune, draws in [("eight_schools", False, 0, 25), ("eight_schools", True, 220, 30), ("radon", True, 130, 10),
+                                     ("std_normal", False, 0, 10)]:
+        spec = models.std_normal(40) if name == "std_normal" else models.BUILDERS[name]()
+        n = spec.n
+        q0 = spec.initial_point() + np.random.default_rng(1).uniform(-1, 1, n)
+        pot = qp.QuadPotentialDiagAdapt(n, q0.copy(), np.ones(n), 10) if adapt else qp.QuadPotentialDiag(np.ones(n))
+        qs, sts, _ = reference_chain(spec, logp_numpy.make_logp(spec), q0, 77, tune, draws, pot, adapt)
+        key = f"diag-{name}-{adapt}-{tune}-{draws}"
+        record(out, key + "/q", qs)
+        for k in PORT_STAT_KEYS:
+            record(out, f"{key}/{k}", [s[k] for s in sts])
+    # QuadPotentialFull, fixed step size
+    spec = models.mvgauss(n=15, seed=2)
+    q0 = np.random.default_rng(3).normal(size=15)
+    qs, _, _ = reference_chain(spec, logp_numpy.make_logp(spec), q0, 5, 0, 12, qp.QuadPotentialFull(spec.data["cov"]), False)
+    record(out, "dense/q", qs)
+    # QuadPotentialFullAdapt (init="adapt_full") through the first window switch for Eight Schools
+    for name, tune, draws in [("eight_schools", 130, 10), ("radon", 60, 5)]:
+        spec = models.BUILDERS[name]()
+        n = spec.n
+        q0 = spec.initial_point() + np.random.default_rng(4).uniform(-1, 1, n)
+        with warnings.catch_warnings():
+            warnings.simplefilter("ignore")
+            pot = qp.QuadPotentialFullAdapt(n, q0.copy(), np.eye(n), 10)
+        qs, sts, step = reference_chain(spec, logp_numpy.make_logp(spec), q0, 91, tune, draws, pot, True)
+        key = f"dense_adapt-{name}"
+        record(out, key + "/q", qs)
+        for k in ("tree_size", "depth", "index_in_trajectory", "energy", "step_size"):
+            record(out, f"{key}/{k}", [s[k] for s in sts])
+        record(out, key + "/cov", step.potential._cov)
+        record(out, key + "/chol", step.potential._chol)
+    # the SURVEY 8c known answer of the loader: Eight Schools from 0, unit mass, seed 20240922
+    spec = models.eight_schools()
+    qs, sts, _ = reference_chain(spec, logp_numpy.make_logp(spec), np.zeros(10), 20240922, 0, 5, qp.QuadPotentialDiag(np.ones(10)),
+                                 False)
+    assert [(s["depth"], s["tree_size"], s["index_in_trajectory"]) for s in sts] == \
+        [(4, 15, -10), (5, 31, -10), (5, 31, -11), (5, 31, 13), (4, 15, 10)], "the reference loader is broken"
+    record(out, "self_check/q", qs)
+    for k in PORT_STAT_KEYS:
+        record(out, f"self_check/{k}", [s[k] for s in sts])
+    np.savez_compressed(os.path.join(OUT, "ref_port_chains.npz"), **out)
+
+
+def step_seam_case():
+    """ref_step_seam.npz: the reference NUTS (default potential) driven like _iter_sample drives a step method, the run
+    tests/test_step_seam.py drives B200NUTS through: positions, every per-draw stat with a value, the stats keys, and where
+    the caller's generator is left."""
+    spec = models.eight_schools()
+    f = logp_numpy.make_logp(spec)
+    q0 = spec.initial_point() + np.random.default_rng(3).uniform(-1, 1, spec.n)
+    start = {v.name: q0[v.offset : v.offset + v.size].copy() for v in spec.vars}
+    ref, _ = ref_loader.make_nuts(f, spec.var_sizes, start, step_rng=0)  # default potential: DiagAdapt(zeros, ones, 10)
+    tune, draws = 60, 25
+    ref.setup_chain(np.random.default_rng(20240922), tune, draws)  # the loop of _iter_sample
+    ref.tune = True
+    ref.reset_tuning()
+    point, qs, sts = dict(start), [], []
+    for i in range(tune + draws):
+        if i == tune:
+            ref.stop_tuning()
+        point, st = ref.step(point)
+        qs.append(np.concatenate([np.ravel(point[k]) for k in start]))
+        sts.append(st[0])
+    qs = np.array(qs)
+    s = ref.rng.bit_generator.state["state"]["state"]
+    out = dict(q=qs, rng_after=np.array([s >> 64, s & (2**64 - 1)], dtype=np.uint64),
+               stats_keys=np.array(sorted(sts[0])), stats_dtypes_shapes_keys=np.array(sorted(type(ref).stats_dtypes_shapes)))
+    for k in ("depth", "tree_size", "index_in_trajectory", "diverging", "reached_max_treedepth", "divergences", "step_size",
+              "step_size_bar", "mean_tree_accept", "energy", "energy_error", "max_energy_error", "model_logp"):
+        out["stat_" + k] = np.array([x[k] for x in sts])
+    np.savez_compressed(os.path.join(OUT, "ref_step_seam.npz"), **out)
+
+
+def potential_objects():
+    """The reference QuadPotential objects tests/test_potentials.py hands to pymc_b200.potentials, keyed by label."""
+    import warnings
+    qp = ref_loader.quadpotential()
+    n = 4
+    rng = np.random.default_rng(0)
+    v, mean = rng.uniform(0.5, 2.0, n), rng.normal(size=n)
+    B = rng.normal(size=(n, n))
+    cov = B @ B.T + n * np.eye(n)
+    objs = {
+        "diag": qp.QuadPotentialDiag(v),
+        "diag_adapt": qp.QuadPotentialDiagAdapt(n, mean, v, 7, adaptation_window=33, discard_window=9),
+        "diag_adapt_exp": qp.QuadPotentialDiagAdaptExp(n, mean, alpha=0.03, use_grads=True, stop_adaptation=120),
+        "diag_adapt_exp_nostop": qp.QuadPotentialDiagAdaptExp(n, mean, alpha=0.03, use_grads=True),
+        "full": qp.QuadPotentialFull(cov),
+        "full_inv": qp.QuadPotentialFullInv(cov),
+        "diag_adapt_early": qp.QuadPotentialDiagAdapt(n, mean, v, 7, early_update=True),
+        "diag_adapt_multiplier": qp.QuadPotentialDiagAdapt(n, mean, v, 7, adaptation_window_multiplier=2),
+        "diag_adapt_exp_nograds": qp.QuadPotentialDiagAdaptExp(n, mean, alpha=0.03),
+        "diag_n3": qp.QuadPotentialDiag(np.ones(3)),
+    }
+    with warnings.catch_warnings():
+        warnings.simplefilter("ignore")
+        objs["full_adapt"] = qp.QuadPotentialFullAdapt(n, mean, np.diag(v), 10, adaptation_window=40,
+                                                       adaptation_window_multiplier=3, update_window=5)
+        objs["full_adapt_offdiag"] = qp.QuadPotentialFullAdapt(n, mean, cov, 10)
+    # the Eight Schools potentials of the whole-run sampler test
+    n = 10
+    rng = np.random.default_rng(1)
+    mean, diag = rng.normal(size=n), rng.uniform(0.5, 2.0, n)
+    objs["es_diag_adapt"] = qp.QuadPotentialDiagAdapt(n, mean, diag, 4, adaptation_window=20, discard_window=5)
+    objs["es_diag"] = qp.QuadPotentialDiag(diag)
+    return objs
+
+
+def potential_cases():
+    """ref_potentials.json: {label: {"__class__": class name, attribute: value}} of the reference QuadPotential objects, every
+    plain-valued attribute (numbers, strings, float arrays as lists); generators and running estimators are left out."""
+    import json
+    out = {}
+    for label, obj in potential_objects().items():
+        d = out[label] = {"__class__": type(obj).__name__}
+        for k, val in vars(obj).items():
+            if isinstance(val, np.ndarray) and val.dtype == np.float64:
+                d[k] = val.tolist()
+            elif isinstance(val, (bool, int, float, str, np.integer, np.floating, np.bool_)):
+                d[k] = val.item() if isinstance(val, np.generic) else val
+    with open(os.path.join(OUT, "ref_potentials.json"), "w") as fh:
+        json.dump(out, fh, indent=1)
+        fh.write("\n")
+
+
 if __name__ == "__main__":
+    if len(sys.argv) > 1 and sys.argv[1] == "seams":
+        port_cases()
+        step_seam_case()
+        potential_cases()
+        raise SystemExit(0)
     if len(sys.argv) > 1 and sys.argv[1] == "lockstep":
         lockstep_cases()
         raise SystemExit(0)

@@ -21,9 +21,9 @@ It restates, function by function, what the reference does for one NUTS transiti
 It performs the same floating-point operations with the same NumPy/BLAS calls in the same order
 and consumes the two per-chain PCG64 streams in the same order (SURVEY.md 8a row a15), so that on
 the same NumPy/SciPy it is *bit-identical* to the reference files loaded verbatim
-(``oracle/ref_loader.py``); ``tests/test_oracle_vs_reference.py`` asserts that whenever
-/root/reference is present, and ``tests/golden/*.npz`` (made by ``oracle/make_golden.py`` from the
-verbatim reference) pin it everywhere else.  PARITY STATUS: pinned.
+(``oracle/ref_loader.py``); ``tests/test_oracle_vs_reference.py`` asserts that against reference
+chains recorded in ``tests/golden/ref_port_chains.npz``, and the other ``tests/golden/*.npz`` (all
+made by ``oracle/make_golden.py`` from the verbatim reference) pin it further.  PARITY STATUS: pinned.
 
 Only tests/, bench.py's cpu_baseline / --impl reference legs and __graft_entry__.smoke() may
 import this module; nothing under pymc_b200/ does.

@@ -6,12 +6,11 @@ but the HMC files themselves run unmodified once a few stub modules stand in for
 (SURVEY.md section 8c).  This module builds those stubs in ``sys.modules`` and executes the
 reference files *from where they lie* under ``/root/reference`` -- nothing is copied.
 
-It is used for exactly two things:
-  * ``oracle/make_golden.py`` -- generating the committed golden vectors in ``tests/golden/``;
-  * ``tests/test_oracle_vs_reference.py`` -- pinning ``oracle/nuts_numpy.py`` (our restatement,
-    which *does* travel to the GPU box) against the true reference, when the reference exists.
+It is used for one thing: ``oracle/make_golden.py`` generates the committed golden vectors in
+``tests/golden/`` with it, among them the recorded reference chains, step-method run and potential
+objects the tests compare with.  The tests themselves never need the reference tree.
 
-``/root/reference`` does not exist on the GPU box: callers must check ``available()`` first.
+Callers must check ``available()`` first.
 Nothing in ``pymc_b200`` imports this file.
 """
 from __future__ import annotations

@@ -1,7 +1,14 @@
-"""Shared helpers: model specs per golden file, GPU replay (free-running and single-draw), oracle replay."""
+"""Shared helpers: model specs per golden file, GPU replay (free-running and single-draw), oracle replay, recorded reference
+potential objects."""
+import json
+import os
+
 import numpy as np
 
 from pymc_b200 import _lib, models
+
+_REF_POTENTIALS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_potentials.json")
+_REF_CLASSES = {}
 
 SPEC_OF = {
     "std_normal_fixed": lambda: models.std_normal(100),
@@ -101,6 +108,19 @@ def gpu_single_draws(cm, d, name, chain=0):
         for k, v in res.stats.items():
             st.setdefault(k, np.zeros(T, dtype=v.dtype))[sel] = v[:, 0]
     return dq, st
+
+
+def reference_potential(label):
+    """One of the reference's QuadPotential objects as ``pymc_b200.potentials`` sees it: an instance of a class with the
+    reference class's name, carrying the plain-valued attributes the reference object had after construction
+    (tests/golden/ref_potentials.json, recorded from the verbatim classes by ``python -m oracle.make_golden seams``)."""
+    with open(_REF_POTENTIALS) as fh:
+        attrs = json.load(fh)[label]
+    name = attrs.pop("__class__")
+    obj = _REF_CLASSES.setdefault(name, type(name, (), {}))()
+    for k, v in attrs.items():
+        setattr(obj, k, np.array(v, dtype=np.float64) if isinstance(v, list) else v)
+    return obj
 
 
 def discrete_equal(st, d, chain):

@@ -44,6 +44,39 @@ def test_roofline_objects():
     json.dumps([r, t])
 
 
+def test_dump_outputs_writes_a_fixed_bounded_sample(tmp_path, monkeypatch):
+    sys.path.insert(0, ROOT)
+    import bench
+    import numpy as np
+    import torch
+
+    from pymc_b200.engine import NutsResult
+
+    C, T, n = 50, 7, 3
+    g = torch.Generator().manual_seed(0)
+    res = NutsResult(draws=torch.randn(C, T, n, generator=g, dtype=torch.float64),
+                     stats={"tree_size": torch.randint(1, 64, (C, T), generator=g, dtype=torch.int32),
+                            "diverging": torch.zeros(C, T, dtype=torch.uint8)},
+                     summary={"grad_evals": torch.arange(C, dtype=torch.int64), "final_var": torch.ones(C, n, dtype=torch.float64)},
+                     kernel_ms=0.0, launches=1, tune=0, n_draws=T, store_warmup=False)
+    bench.dump_outputs(res, str(tmp_path / "all"))
+    out = {p.stem: np.load(p) for p in (tmp_path / "all").iterdir()}
+    assert set(out) == {"chains", "draws", "stat_tree_size", "stat_diverging", "summary_grad_evals", "summary_final_var"}
+    assert all(a.dtype == np.float64 for a in out.values())
+    assert np.array_equal(out["chains"], np.arange(C)) and np.array_equal(out["draws"], res.draws.numpy())
+    assert np.array_equal(out["stat_tree_size"], res.stats["tree_size"].numpy())
+    # above the cap: the same seeded chains in every array, and no more bytes than the cap
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4096 * 6 + 10 * 8 * (T * n + 2 * T + 1 + n + 1))
+    for d in ("a", "b"):
+        bench.dump_outputs(res, str(tmp_path / d))
+    a = {p.stem: np.load(p) for p in (tmp_path / "a").iterdir()}
+    b = {p.stem: np.load(p) for p in (tmp_path / "b").iterdir()}
+    idx = a["chains"].astype(int)
+    assert len(idx) == 10 and np.all(np.diff(idx) > 0) and all(np.array_equal(a[k], b[k]) for k in a)
+    assert np.array_equal(a["draws"], res.draws.numpy()[idx]) and np.array_equal(a["summary_grad_evals"], idx)
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= bench.DUMP_BYTES
+
+
 def test_reference_arm_prints_the_contract_line():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0",
                           "--cpu-chains", "2", "--tune", "6", "--draws", "8"], capture_output=True, text=True, timeout=600, cwd=ROOT)

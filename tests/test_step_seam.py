@@ -1,5 +1,6 @@
 """Seam B3 (SURVEY 8b): ``B200NUTS`` driven exactly like ``_iter_sample`` drives a step method
-(pymc/sampling/mcmc.py:1503-1578), against the VERBATIM reference ``NUTS`` on the same generator.
+(pymc/sampling/mcmc.py:1503-1578), against the VERBATIM reference ``NUTS`` on the same generator (its run recorded in
+tests/golden/ref_step_seam.npz by ``python -m oracle.make_golden seams``).
 
 CPU: the device engine is replaced by a stand-in with the ``CompiledModel.nuts_run`` interface that runs the oracle
 (bit-identical to the reference, tests/test_oracle_vs_reference.py), which pins the protocol glue: stream derivation
@@ -8,11 +9,8 @@ import numpy as np
 import pytest
 
 from b200_helpers import OracleEngine
-from oracle import logp_numpy, ref_loader
 from pymc_b200 import models
 from pymc_b200.step import B200NUTS
-
-needs_reference = pytest.mark.skipif(not ref_loader.available(), reason="/root/reference is not present")
 
 
 def drive(step, start, rng, tune, draws):
@@ -30,29 +28,28 @@ def drive(step, start, rng, tune, draws):
     return np.array(out), stats
 
 
-@needs_reference
-def test_b200nuts_protocol_matches_reference_nuts_with_oracle_engine():
+def test_b200nuts_protocol_matches_reference_nuts_with_oracle_engine(golden):
     spec = models.eight_schools()
-    f = logp_numpy.make_logp(spec)
     q0 = spec.initial_point() + np.random.default_rng(3).uniform(-1, 1, spec.n)
     start = {v.name: q0[v.offset : v.offset + v.size].copy() for v in spec.vars}
     tune, draws, seed = 60, 25, 20240922
 
-    ref, _ = ref_loader.make_nuts(f, spec.var_sizes, start, step_rng=0)  # default potential: DiagAdapt(zeros, ones, 10)
-    want_q, want_st = drive(ref, dict(start), np.random.default_rng(seed), tune, draws)
-    rng_ref_after = ref.rng.bit_generator.state["state"]["state"]
+    # the reference NUTS with its default potential, DiagAdapt(zeros, ones, 10), driven by drive() from default_rng(seed)
+    want = golden("ref_step_seam")
+    hi, lo = (int(x) for x in want["rng_after"])
+    rng_ref_after = (hi << 64) | lo
 
     mine = B200NUTS(OracleEngine(spec))
     rng = np.random.default_rng(seed)
     got_q, got_st = drive(mine, dict(start), rng, tune, draws)
 
-    assert np.array_equal(got_q, want_q)
+    assert np.array_equal(got_q, want["q"])
     for k in ("depth", "tree_size", "index_in_trajectory", "diverging", "reached_max_treedepth", "divergences"):
-        assert [s[k] for s in got_st] == [w[k] for w in want_st], k
+        assert [s[k] for s in got_st] == want["stat_" + k].tolist(), k
     for k in ("step_size", "step_size_bar", "mean_tree_accept", "energy", "energy_error", "max_energy_error", "model_logp"):
-        np.testing.assert_allclose([s[k] for s in got_st], [w[k] for w in want_st], rtol=1e-12, atol=1e-12, err_msg=k)
-    assert set(B200NUTS.stats_dtypes_shapes) == set(type(ref).stats_dtypes_shapes)
-    assert set(got_st[0]) == set(want_st[0])
+        np.testing.assert_allclose([s[k] for s in got_st], want["stat_" + k], rtol=1e-12, atol=1e-12, err_msg=k)
+    assert set(B200NUTS.stats_dtypes_shapes) == set(want["stats_dtypes_shapes_keys"].tolist())
+    assert set(got_st[0]) == set(want["stats_keys"].tolist())
     # the caller's generator is left exactly where the reference leaves its own
     assert rng.bit_generator.state["state"]["state"] == rng_ref_after
     # shape of a point entry is preserved, other keys pass through

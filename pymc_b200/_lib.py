@@ -11,7 +11,7 @@ import os
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("B200_LIB", os.path.join(_HERE, "libb200nuts.so"))  # override: A/B builds while tuning
+LIB_PATH = os.path.join(_HERE, "libb200nuts.so")
 
 MEM_HOST, MEM_DEVICE = 0, 1
 MASS_DIAG, MASS_DIAG_ADAPT, MASS_DENSE, MASS_DIAG_ADAPT_GRAD, MASS_DENSE_ADAPT = 0, 1, 2, 3, 4
@@ -259,15 +259,12 @@ def load() -> C.CDLL:
             raise B200Error(f"{LIB_PATH} is missing: build the CUDA engine first (./build.sh); there is no CPU fallback")
         lib = C.CDLL(LIB_PATH)
         for name, restype, argtypes in SYMBOLS:
-            if name in ("b200_struct_size", "b200_model_set_precision", "b200_model_set_transforms",
-                        "b200_model_set_dense_mass", "b200_pointwise_loglik") and not hasattr(lib, name):
-                continue  # an A/B build (B200_LIB=...) older than ABI 0.2.0; tests/test_abi.py requires it of the in-tree library
             fn = getattr(lib, name)
             fn.restype = restype
             fn.argtypes = argtypes
         mirrors = [ModelDesc, NutsCfg, Stats, ChainSummary, Pcg64State, Ir, IrVar, IrPrior, IrTerm, IrLik, IrAr1, IrParam, IrFactor,
                    ChainStateC]
-        for which, cls in enumerate(mirrors if hasattr(lib, "b200_struct_size") else []):
+        for which, cls in enumerate(mirrors):
             if lib.b200_struct_size(which) != C.sizeof(cls):
                 raise B200Error(f"ABI mismatch: {cls.__name__} is {C.sizeof(cls)} bytes here, {lib.b200_struct_size(which)} in "
                                 f"{LIB_PATH} (rebuild with ./build.sh)")

@@ -555,10 +555,6 @@ static int npl_team(int n) {
         if (need <= o) return o;
     return 0;
 }
-static bool env_flag(const char* name) {
-    const char* v = getenv(name);
-    return v && v[0] && v[0] != '0';
-}
 
 // Calls f.template operator()<Model, NPL, W>(params) for the model's kind and size.
 template <class F>
@@ -583,7 +579,7 @@ static int dispatch(const b200_model* m, F&& f) {
     }
     switch (m->kind) {
         case B200_MODEL_STD_NORMAL:
-            if (m->n <= 256 && !env_flag("B200_FORCE_TEAM")) { B200_WARP(StdNormalModel, m->std_normal) }
+            B200_WARP(StdNormalModel, m->std_normal)  // n <= 256
             B200_TEAM(StdNormalModel, m->std_normal)
             return fail("std_normal: n=%d exceeds 4096", m->n);
         case B200_MODEL_EIGHT_SCHOOLS:
@@ -596,7 +592,7 @@ static int dispatch(const b200_model* m, F&& f) {
             B200_TEAM(StochVolModel, m->stochvol)
             return fail("stochvol: n=%d exceeds 4096", m->n);
         case B200_MODEL_IR:
-            if (m->n <= 256 && !env_flag("B200_FORCE_TEAM")) { B200_WARP(IrModel, m->ir) }
+            B200_WARP(IrModel, m->ir)  // n <= 256
             B200_TEAM(IrModel, m->ir)
             return fail("ir: n=%d exceeds the chain-per-CTA limit (4096)", m->n);
     }
@@ -661,7 +657,7 @@ static int stage_in(Staged& s, const void* user, size_t bytes, int mem, bool cop
     s.bytes = bytes;
     s.host = (mem == B200_MEM_HOST) && user != nullptr;
     s.out = copy_out;
-    if (s.host && direct && !copy_in && !getenv("B200_NO_DIRECT_HOST_WRITES")) {
+    if (s.host && direct && !copy_in) {
         cudaPointerAttributes at{};
         if (cudaPointerGetAttributes(&at, user) == cudaSuccess && at.type == cudaMemoryTypeHost && at.devicePointer) {
             s.user = at.devicePointer;
@@ -679,11 +675,6 @@ static int stage_in(Staged& s, const void* user, size_t bytes, int mem, bool cop
 static int stage_out(Staged& s, cudaStream_t st) {
     if (s.host && s.out) CU(cudaMemcpyAsync(s.user, s.dptr(), s.bytes, cudaMemcpyDeviceToHost, st));
     return 0;
-}
-
-static int env_int(const char* name, int dflt) {
-    const char* v = getenv(name);
-    return v ? atoi(v) : dflt;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -973,7 +964,7 @@ static int launch_logistic(const b200_model* m, int C, const double* Q, long lon
     auto kern = logistic_fused_kernel<KB>;
     const size_t smem = logistic_smem_bytes<KB>();
     CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<dim3(bs.gx, bs.cpad / kLogiChains), 32 * (kLogiChains / (8 * B200_LOGI_MB)), smem, st>>>(m->X, m->y8, m->n_rows, Q, ldq, C, m->n, bs.gpart.as<double>(),
+    kern<<<dim3(bs.gx, bs.cpad / kLogiChains), 32 * (kLogiChains / (8 * kLogiMB)), smem, st>>>(m->X, m->y8, m->n_rows, Q, ldq, C, m->n, bs.gpart.as<double>(),
                                                                bs.lpart.as<double>(), bs.cpad);
     CU(cudaGetLastError());
     return 0;
@@ -1014,17 +1005,10 @@ static int batch_eval(b200_model* m, int C, const double* Q, double* G, double* 
         if (m->KP != kTcK) {  // partials are [.][.][KP]: the tensor-core kernel writes 128-wide rows
             return fail("tensor-core mode needs the 128-feature layout (65..128 features); this model has %d", m->n);
         }
-        if (env_int("B200_LOGI_TC_V", 2) == 1) {  // version 1 of the kernel (8 epilogue warps, drains through global memory)
-            auto kern = logistic_tc_kernel;
-            CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTcSmemBytes));
-            LogisticTcArgs A{m->y8, m->n_rows, m->tc_slabs, Q, ld, C, m->n, bs.gpart.as<double>(), bs.lpart.as<double>(), bs.cpad};
-            kern<<<dim3(bs.gx, bs.cpad / kLogiChains), kTcThreads, kTcSmemBytes, st>>>(m->map_hi, m->map_lo, A);
-        } else {
-            auto kern = logistic_tc2_kernel;
-            CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTc2SmemBytes));
-            LogisticTc2Args A{m->y32, m->n_rows, m->tc_slabs, Q, ld, C, m->n, bs.gpart.as<double>(), bs.lpart.as<double>(), bs.cpad};
-            kern<<<dim3(bs.gx, bs.cpad / kLogiChains), kTc2Threads, kTc2SmemBytes, st>>>(m->map_hi, m->map_lo, A);
-        }
+        auto kern = logistic_tc2_kernel;
+        CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTc2SmemBytes));
+        LogisticTc2Args A{m->y32, m->n_rows, m->tc_slabs, Q, ld, C, m->n, bs.gpart.as<double>(), bs.lpart.as<double>(), bs.cpad};
+        kern<<<dim3(bs.gx, bs.cpad / kLogiChains), kTc2Threads, kTc2SmemBytes, st>>>(m->map_hi, m->map_lo, A);
         CU(cudaGetLastError());
     } else
     switch (m->KP) {
@@ -1064,6 +1048,9 @@ static int lockstep_logp(b200_model* m, const double* q_dev, int C, double* logp
     return 0;
 }
 
+// warps per chain of the lock-step advance kernel for long state vectors (n > 512): 16 is 5 % faster than 8 at n = 10^4
+static constexpr int kLsAdvW = 16;
+
 // The lock-step driver: advance <-> batched evaluation until every chain is done.
 static int run_lockstep(b200_model* m, LsDev P, cudaStream_t st) {
     const int C = P.C, n = P.n;
@@ -1078,9 +1065,12 @@ static int run_lockstep(b200_model* m, LsDev P, cudaStream_t st) {
     auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
     const size_t b_state = up((size_t)C * sizeof(LsState)), b_vecs = up((size_t)C * P.vec_stride * sizeof(double)), b_mat = up(mat);
     const size_t b_l = up((size_t)C * sizeof(double)), b_cnt = up(4 * sizeof(int)), b_mom = up((size_t)C * sizeof(int));
-    // compaction of the request rows once finished chains free a whole tile of them (lockstep.cuh: ls_compact_*)
-    const int ctile = std::max(1, env_int("B200_LS_COMPACT_TILE", 128));
-    const bool compact = env_int("B200_LS_COMPACT", 1) != 0 && C > ctile;
+    // compaction of the request rows once finished chains free a whole tile (128 rows) of them (lockstep.cuh: ls_compact_*).
+    // B200_LS_COMPACT_TILE is a test seam, not a tuning option: 0 never compacts, and a small tile makes runs of a few dozen
+    // chains compact, so that a test can check that compaction changes no result.
+    const char* tile_env = getenv("B200_LS_COMPACT_TILE");
+    const int ctile = tile_env ? atoi(tile_env) : 128;
+    const bool compact = ctile > 0 && C > ctile;
     const int n_mats = (dense ? 8 : 2) + (compact ? 1 : 0);
     // DENSE_ADAPT: four n x n matrices per chain (covariance, Cholesky factor, two raw scatter matrices; dense_adapt.cuh)
     const bool fa = P.mass_kind == B200_MASS_DENSE_ADAPT;
@@ -1137,8 +1127,8 @@ static int run_lockstep(b200_model* m, LsDev P, cudaStream_t st) {
     // requesting rows (for n = 10^4 they cost as much as the gradient and mass GEMMs of ALL chains), so requests are queued on
     // the device and served in batches: when half of the live chains are waiting in the queue, or as soon as a chain reaches
     // the end of its draw without its momentum (it then idles for one round: LsState phase 3).  The noise z of (chain, draw)
-    // does not depend on when it is served, so results are identical for every threshold.  B200_LS_MOM_DEFER=0: serve every round.
-    const double defer = fa ? 0.0 : std::max(0.0, std::min(1.0, env_int("B200_LS_MOM_DEFER", 50) / 100.0));
+    // does not depend on when it is served, so results are identical for every threshold.
+    const double defer = fa ? 0.0 : 0.5;
     CU(cudaMemsetAsync(P.counters, 0, 4 * sizeof(int), st));
     int C_eval = C;             // rows of the request matrices in use (shrinks when finished chains free a tile)
     for (;;) {
@@ -1170,10 +1160,7 @@ static int run_lockstep(b200_model* m, LsDev P, cudaStream_t st) {
             }
         }
         CU(cudaMemsetAsync(P.counters, 0, 2 * sizeof(int), st));
-#ifndef B200_ADV_W
-#define B200_ADV_W 16  // warps per chain of the lock-step advance kernel for long state vectors (16: 5 % faster than 8 at n = 10^4)
-#endif
-        if (n > 512) ls_advance_kernel<B200_ADV_W><<<C, 32 * B200_ADV_W, 0, st>>>(P);
+        if (n > 512) ls_advance_kernel<kLsAdvW><<<C, 32 * kLsAdvW, 0, st>>>(P);
         else ls_advance_kernel<1><<<blocks, 128, 0, st>>>(P);
         CU(cudaGetLastError());
         ++launches;
@@ -1204,11 +1191,9 @@ struct NutsLaunch {
     template <class Model, int NPL, int W>
     int operator()(const typename Model::Params& MP) {
         constexpr int NP = 32 * W * NPL;
-        constexpr bool SUBS = (W > 1) ? true : (B200_SUBTREE_SMEM != 0);
-        int wpb = (W == 1) ? env_int("B200_NUTS_WPB", 8) : 1;  // chains per CTA (8 warps, 1 CTA per SM: measured best, r2)
-        int hot = env_int("B200_NUTS_HOT", (W == 1) ? 2 : 1);
-        wpb = std::max(1, std::min(wpb, B200_NUTS_THREADS / 32));
-        hot = std::max(0, std::min(hot, P.max_td));
+        constexpr bool SUBS = (W > 1);  // nuts_warp_kernel's default
+        const int wpb = (W == 1) ? kNutsWarpChains : 1;  // chains per CTA
+        int hot = std::min((W == 1) ? 2 : 1, P.max_td);
         const size_t data = (Model::shared_bytes(MP) + 15) & ~(size_t)15;
         size_t smem = data + (size_t)wpb * nuts_warp_smem_bytes(NP, hot, SUBS, W);
         while (smem > 227 * 1024 && hot > 0) {  // shrink the hot window until the CTA fits
@@ -1229,7 +1214,7 @@ struct NutsLaunch {
         P.done = reinterpret_cast<int*>(base + tree_bytes + ctx_bytes);
         P.ticket = reinterpret_cast<unsigned int*>(P.done + P.C);
         CU(cudaMemsetAsync(P.done, 0, sched_bytes, st));
-        auto kern = nuts_warp_kernel<Model, NPL, W, SUBS>;
+        auto kern = nuts_warp_kernel<Model, NPL, W>;
         CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         // persistent grid: every CTA resident (teams take (chain, segment) units from the ticket counter)
         const int threads = (W == 1) ? wpb * 32 : 32 * W;
@@ -1241,8 +1226,7 @@ struct NutsLaunch {
         // iterations per work unit: fine enough to balance chains of different cost, coarse enough that the ~3 KB state
         // hand-over per unit is noise.  One unit per chain when every chain has its own resident team anyway.
         const int Ttot = P.n_iter;
-        int seg = env_int("B200_NUTS_SEG", 50);  // measured (r2): 10 -> 390 ms, 25 -> 370, 50 -> 361, 100 -> 367
-        if (seg <= 0 || need <= blocks) seg = Ttot;
+        const int seg = (need <= blocks) ? Ttot : 50;  // 50 measured (r2): 10 -> 390 ms, 25 -> 370, 50 -> 361, 100 -> 367
         P.seg_iters = std::max(1, std::min(seg, Ttot));
         typename Model::Params MPl;
         if (launch_params<Model>(m, MP, (long long)blocks * wpb, &MPl)) return -1;
@@ -1358,11 +1342,10 @@ extern "C" int b200_nuts_run(b200_model* m, const b200_nuts_cfg* cfg, const doub
         // 12 x C x T single-value PCIe write transactions (24 M for the Radon bench), which costs more link time than the
         // draws themselves.  They are staged in HBM (one arena in the model handle) and leave with 12 DMA copies at the end
         // (143 MB for the Radon bench).  The draws -- 256-byte coalesced row segments -- keep the direct path.
-        const bool direct_stats = getenv("B200_DIRECT_STATS") != nullptr;
 #define B200_ST(i, field, type)                                                              \
     if (stats->field) {                                                                      \
-        if (!direct_stats) lend(st_arr[i], stats->field, ct * sizeof(type));                 \
-        if (stage_in(st_arr[i], stats->field, ct * sizeof(type), mem, false, true, st, /*direct=*/direct_stats)) return -1; \
+        lend(st_arr[i], stats->field, ct * sizeof(type));                                    \
+        if (stage_in(st_arr[i], stats->field, ct * sizeof(type), mem, false, true, st)) return -1; \
         ds.field = (type*)st_arr[i].ptr();                                                   \
     }
         B200_ST(0, depth, int32_t) B200_ST(1, tree_size, int32_t) B200_ST(2, index_in_trajectory, int32_t)

@@ -154,11 +154,10 @@ __host__ __device__ constexpr size_t logistic_smem_bytes() {
     return ((size_t)kLogiChains * (8 * KB + 4) + 2 * (size_t)kLogiRows * (8 * KB + 4)) * sizeof(double) + 64;
 }
 
-#ifndef B200_LOGI_MB
-#define B200_LOGI_MB 1  // 8-chain accumulator blocks per warp: 1 -> 16 warps x 8 chains per CTA (126 regs, 4 warps per scheduler:
-                        // 10.8 ms per 512-chain batch), 2 -> 8 warps x 16 chains (212 regs, 12.4 ms)
-#endif
-template <int KB, int MB = B200_LOGI_MB>
+// 8-chain accumulator blocks per warp: 1 -> 16 warps x 8 chains per CTA (126 regs, 4 warps per scheduler: 10.8 ms per
+// 512-chain batch) is faster than 2 -> 8 warps x 16 chains (212 regs, 12.4 ms)
+constexpr int kLogiMB = 1;
+template <int KB, int MB = kLogiMB>
 __global__ void __launch_bounds__(32 * (kLogiChains / (8 * MB)), 1)
     logistic_fused_kernel(const double* __restrict__ X /*[Npad][8KB]*/, const uint8_t* __restrict__ y, long long N,
                           const double* __restrict__ Q, long long ldq, int C, int K,

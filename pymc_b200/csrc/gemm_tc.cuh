@@ -42,18 +42,11 @@ __device__ __forceinline__ void tc_ld8(uint32_t taddr, uint32_t (&v)[8]) {
 // every drained value to fp64 (F2F.F64.F32 + DADD): ncu (profiles/r2_tc_gemm_tc_*) showed the tensor pipe 27 % busy and the
 // kernel waiting on exactly those two opcodes (22 % of the instructions each, 47 % of the stall samples) with a quarter of the
 // accumulators spilled -- the conversion unit, not the MMAs or L2 (40 % of the LTS cap), set the pace.
-#ifndef B200_GT_KAHAN
-#define B200_GT_KAHAN 1  // 0: plain round-to-nearest fp32 sums (72 registers instead of 144, one FADD per value)
-#endif
 __device__ __forceinline__ void kahan_add(float& s, float& c, float x) {
-#if B200_GT_KAHAN
     const float y = x - c;
     const float t = s + y;
     c = (t - s) - y;
     s = t;
-#else
-    s += x;
-#endif
 }
 
 struct GemmTcArgs {

@@ -29,12 +29,7 @@ namespace b200 {
 constexpr int kLsLevels = 12;
 
 // the O(n) vector passes of the advance kernel are latency-bound strided loops: unrolling keeps several loads in flight
-#ifndef B200_LS_UNROLL_N
-#define B200_LS_UNROLL_N 4
-#endif
-#define B200_LS_PRAGMA(x) _Pragma(#x)
-#define B200_LS_UNROLL_(n) B200_LS_PRAGMA(unroll n)
-#define B200_LS_UNROLL B200_LS_UNROLL_(B200_LS_UNROLL_N)
+constexpr int kLsUnroll = 4;
 
 // A pass over a chain's vectors in tiles of U elements per thread: ALL loads of a tile, then the arithmetic and the stores.
 // Written as `for (i) { load; store; }` the compiler must keep every load behind the previous iteration's store (the vectors
@@ -111,7 +106,7 @@ struct LsDev {
 // thread of the team (common.cuh), so every thread carries an identical private copy of the scalar state.
 template <int W>
 __global__ void __launch_bounds__(W == 1 ? 128 : 32 * W) ls_advance_kernel(const LsDev P) {
-    constexpr int TS = 32 * W, U = B200_LS_UNROLL_N;
+    constexpr int TS = 32 * W, U = kLsUnroll;
     __shared__ double red_s[W == 1 ? 1 : 8 * W];
     double* red = red_s;
     const int lane = (W == 1) ? (threadIdx.x & 31) : (int)threadIdx.x;  // index inside the team
@@ -138,7 +133,7 @@ __global__ void __launch_bounds__(W == 1 ? 128 : 32 * W) ls_advance_kernel(const
     auto req_logp = [&]() -> double {
         if (P.logp_from_dot) {
             double s = 0.0;
-            B200_LS_UNROLL
+#pragma unroll kLsUnroll
             for (int i = lane; i < n; i += TS) s = fma(qreq[i], greq[i], s);
             return P.logp_const + 0.5 * team_sum<W>(s, lane, red);
         }
@@ -153,7 +148,7 @@ __global__ void __launch_bounds__(W == 1 ? 128 : 32 * W) ls_advance_kernel(const
     } else if (S.phase == 0) {
         // ---- evaluation at q0 has arrived: the start state of the first draw --------------------------------
         S.cur_logp = req_logp();
-        B200_LS_UNROLL
+#pragma unroll kLsUnroll
         for (int i = lane; i < n; i += TS) {
             V(LV_Q)[i] = qreq[i];
             V(LV_G)[i] = greq[i];
@@ -415,7 +410,7 @@ __global__ void __launch_bounds__(W == 1 ? 128 : 32 * W) ls_advance_kernel(const
                 const int tm = S.fg_m, tv = S.fg_v;
                 S.fg_m = S.bg_m; S.fg_v = S.bg_v; S.fg_n = S.bg_n;
                 S.bg_m = tm; S.bg_v = tv; S.bg_n = 0.0;
-                B200_LS_UNROLL
+#pragma unroll kLsUnroll
                 for (int i = lane; i < n; i += TS) { V(S.bg_m)[i] = 0.0; V(S.bg_v)[i] = 0.0; }
             }
             ++S.k_samples;
@@ -466,7 +461,7 @@ __global__ void __launch_bounds__(W == 1 ? 128 : 32 * W) ls_advance_kernel(const
                                 [&](int u, int i) { p[i] = a_[u]; v[i] = b_[u]; kin = fma(a_[u], b_[u], kin); });
             } else {
                 const double* var = V(LV_VAR);
-                B200_LS_UNROLL
+#pragma unroll kLsUnroll
                 for (int i = lane; i < n; i += TS) {
                     const double zz = (P.momentum_source == B200_MOMENTUM_HOST_BUFFER)
                                           ? P.z[((long long)chain * Ttot + S.it) * n + i]
@@ -484,7 +479,7 @@ __global__ void __launch_bounds__(W == 1 ? 128 : 32 * W) ls_advance_kernel(const
             for (int t = S.it; t < Ttot; ++t) {
                 if (!(P.store_warmup || t >= P.tune)) continue;
                 const int t_o = P.store_warmup ? t : t - P.tune;
-                B200_LS_UNROLL
+#pragma unroll kLsUnroll
                 for (int i = lane; i < n; i += TS) P.draws_out[((long long)chain * T_out + t_o) * n + i] = nan("");
                 if (lane == 0) stats_sentinel(P.st, (long long)chain * T_out + t_o);
             }
@@ -577,7 +572,7 @@ __global__ void __launch_bounds__(W == 1 ? 128 : 32 * W) ls_advance_kernel(const
         *SP = S;
     }
     if (S.phase == 2 && P.sm.final_var)
-        B200_LS_UNROLL
+#pragma unroll kLsUnroll
         for (int i = lane; i < n; i += TS) P.sm.final_var[(long long)chain * n + i] = V(LV_VAR)[i];
     if (S.phase == 2 && fa && P.sm.final_cov) {
         const long long nn = (long long)n * n;

@@ -5,20 +5,20 @@
 // tcgen05 has no fp64 kind, so every fp64 operand is split into two fp16 pieces, v = hi + lo with hi = fp16(v) and
 // lo = fp16(v - hi) (22 significant bits; absolute floor 2^-25 where lo is subnormal), and a product is evaluated as
 // hi*hi + hi*lo + lo*hi in three kind::f16 MMAs with fp32 accumulation (the lo*lo term is below 2^-22 relative).
-// fp32 accumulators only ever cover one slab: X beta sums K = 128 terms, and the gradient accumulator in TMEM is drained
-// into fp64 after every 128-row slab, so neither fp32 rounding nor the tensor cores' one-sided accumulate rounding builds up.
+// fp32 accumulators only ever cover a few slabs: X beta sums K = 128 terms, and the gradient accumulator in TMEM is drained
+// into fp64 every kTcDrain 128-row slabs, so neither fp32 rounding nor the tensor cores' one-sided accumulate rounding builds up.
 // Accuracy against the fp64 path is measured by tests/test_gpu_tc.py and reported in profiles/ (parity report).  The fp64
 // DMMA kernel stays the parity mode.
 //
 // One CTA = 128 chains x a strided set of 128-row slabs of X.  Per slab (FlashAttention-shaped, P kept in TMEM):
-//   TMA   : X_hi, X_lo slab [128 rows][128 features] fp16 -> smem (SWIZZLE_128B, two 64-column boxes each), 2 stages
+//   TMA   : X_hi, X_lo slab [128 rows][128 features] fp16 -> smem (SWIZZLE_128B, two 64-column boxes each) and the slab's
+//           128 labels (fp32), 2 stages
 //   GEMM 1: D1[c][i] = sum_k beta[c][k] X[i][k]     A = beta pieces (smem, K-major), B = X pieces (smem, K-major)
-//   epilog: thread c (TMEM lane c) reads its 128 eta values (tcgen05.ld), computes r = y - sigmoid(eta) and the
+//   epilog: thread c (TMEM lane c) reads its eta values (tcgen05.ld), computes r = y - sigmoid(eta) and the
 //           log-likelihood terms in fp32, splits r into fp16 pieces and writes them back to TMEM (tcgen05.st)
 //   GEMM 2: D2[c][k] += sum_i r[c][i] X[i][k]        A = r pieces (TMEM), B = the SAME X bytes read MN-major
-// Warp roles: warp 0 = TMA producer, warp 1 = MMA issuer (one elected lane), warps 2..9 = epilogue (two per TMEM
-// subpartition, 64 rows of the slab each: the elementwise sigmoid / softplus work is what bounds the kernel, so it gets two
-// warps per scheduler).  D1 is double-buffered so GEMM 1 of slab s+1 runs under the epilogue of slab s.
+// Warp roles: warp 0 = TMA producer, warp 1 = MMA issuer (one elected lane), warps 2..17 = epilogue (four per TMEM
+// subpartition, 32 rows of the slab each).  D1 is double-buffered so GEMM 1 of slab s+1 runs under the epilogue of slab s.
 // TMEM columns (512): D1[0] 0..127, D1[1] 128..255, D2 256..383, r_hi 384..447, r_lo 448..511.
 #pragma once
 #include <cuda.h>
@@ -32,13 +32,10 @@ constexpr int kTcRows = 128;      // rows of X per slab (N of GEMM 1, K of GEMM 
 constexpr int kTcChains = 128;    // chains per CTA (M of both GEMMs = TMEM lanes)
 constexpr int kTcK = 128;         // features (padded)
 constexpr int kTcStages = 2;      // X slab stages in shared memory
-constexpr int kTcThreads = 320;   // 10 warps: TMA producer, MMA issuer, 8 epilogue
-constexpr int kTcEpiThreads = 256;
 constexpr int kTcDrain = 2;       // slabs per fp32 gradient accumulation chunk (16 full-magnitude accumulate steps)
 constexpr uint32_t kTcBlockBytes = kTcRows * 64 * 2;          // one [128 rows][64 cols] fp16 box = 16 KB
 constexpr uint32_t kTcPieceBytes = 2 * kTcBlockBytes;         // one piece of a [128][128] tile = 32 KB
 constexpr uint32_t kTcStageBytes = 2 * kTcPieceBytes;         // X_hi + X_lo = 64 KB
-constexpr size_t kTcSmemBytes = 1024 /*align*/ + 2 * kTcPieceBytes /*beta hi, lo*/ + kTcStages * kTcStageBytes + 256 /*barriers*/;
 
 // ---- raw PTX wrappers ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ void tc_mbar_arrive(uint64_t* bar) {
@@ -91,30 +88,8 @@ __device__ __forceinline__ void tc_mma_ts(uint32_t d_tmem, uint32_t a_tmem, uint
         "r"(a_tmem), "l"(b_desc), "r"(idesc), "r"(accumulate)
         : "memory");
 }
-// 32 consecutive TMEM columns of this thread's lane -> 32 registers
-__device__ __forceinline__ void tc_ld32(uint32_t taddr, uint32_t (&v)[32]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-          "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]), "=r"(v[17]), "=r"(v[18]),
-          "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]),
-          "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-        : "r"(taddr)
-        : "memory");
-}
 __device__ __forceinline__ void tc_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ void tc_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-// 16 registers -> 16 consecutive TMEM columns of this thread's lane
-__device__ __forceinline__ void tc_st16(uint32_t taddr, const uint32_t (&v)[16]) {
-    asm volatile(
-        "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
-        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};" ::"r"(taddr),
-        "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]), "r"(v[9]), "r"(v[10]),
-        "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15])
-        : "memory");
-}
 
 // shared-memory matrix descriptor (cute::UMMA::SmemDescriptor, mma_sm100_desc.hpp): start address, leading / stride byte
 // offsets (all >> 4), version 1 (Blackwell) at bit 46, layout type SWIZZLE_128B = 2 at bits 61..63
@@ -134,293 +109,32 @@ __device__ __forceinline__ uint32_t tc_tile_off(int r, int k) {
     return (uint32_t)(blk * kTcBlockBytes + r * 128 + ((((kk >> 3) ^ (r & 7)) << 4) | ((kk & 7) << 1)));
 }
 
-struct LogisticTcArgs {
-    const uint8_t* y;        // [N]
-    long long N;             // true rows
-    long long n_slabs;       // ceil(N / 128); X pieces are allocated with n_slabs * 128 rows (zero padded)
-    const double* Q;         // [C][ldq] beta per chain
-    long long ldq;
-    int C, K;
-    double* Gpart;           // [gridDim.x][128 features][Cpad]  (feature-major, see the drain)
-    double* lpart;           // [gridDim.x][Cpad]
-    int Cpad;
-};
-
+// logistic_tc2_kernel.  The elementwise sigmoid / softplus work of the epilogue bounds this kernel, not the tensor pipe (a
+// design with 8 epilogue warps that drained into global memory kept the tensor pipe 14 % busy, at 63 warp-instructions per
+// (row, chain) element and 42 % of the stall samples on long-scoreboard waits: profiles/r2_tc_logistic_tc_ncu_summary.csv),
+// so everything around the two GEMMs is shaped to keep the epilogue short:
+//   * 16 epilogue warps (four per TMEM subpartition, 32 rows of the slab each): 4 warps per scheduler hide the TMEM-load and
+//     MUFU latencies that 2 could not;
+//   * the gradient partials stay in REGISTERS as fp64 (32 per thread) across the drains and are written once at the end
+//     (adding every drain into global memory is 2 x 64 read-modify-writes per thread every 2 slabs = 2 GB of L2 traffic per
+//     launch, the long-scoreboard stalls);
+//   * y travels with the slab: the TMA producer copies the slab's 128 labels (fp32, 512 B) into the stage next to the X
+//     pieces, so the element loop neither reads global memory nor converts bytes to floats;
+//   * elementwise math on the MUFU units directly (ex2 / rcp / lg2 .approx.ftz): 12 instructions per element for
+//     sigmoid + softplus + log-likelihood + residual; fp16 pieces of the residual are packed in place;
+//   * rows past N need no masking: their X rows are zero, so eta = 0 exactly, the residual multiplies zero rows in GEMM 2, and
+//     the log-likelihood they add (-softplus(0) each) is added back per slab.
 // Accumulation order and drain period are dictated by the tensor cores' fp32 accumulate, which rounds toward zero: every
 // tcgen05.mma into an accumulator of magnitude |D| loses ~2^-25 |D| one-sidedly (measured, round 2 call 3: 24 accumulate
 // steps per slab -> 8e-7, 384 steps -> 7.9e-6 relative).  So (i) the small correction products hi*lo and lo*hi are issued
 // FIRST, while the accumulator is still tiny, and hi*hi last: 8 full-magnitude steps per GEMM instead of 24; (ii) the
 // gradient accumulator is drained into fp64 every kTcDrain = 2 slabs.
-__global__ void __launch_bounds__(kTcThreads, 1)
-    logistic_tc_kernel(const __grid_constant__ CUtensorMap map_hi, const __grid_constant__ CUtensorMap map_lo, const LogisticTcArgs A) {
-    extern __shared__ char tc_smem_raw[];
-    char* base = reinterpret_cast<char*>((reinterpret_cast<uintptr_t>(tc_smem_raw) + 1023) & ~(uintptr_t)1023);
-    char* beta_s = base;                                   // [hi | lo] pieces, 32 KB each
-    char* x_s = base + 2 * kTcPieceBytes;                  // stages x [X_hi | X_lo]
-    uint64_t* bars = reinterpret_cast<uint64_t*>(x_s + kTcStages * kTcStageBytes);
-    uint64_t* x_full = bars;          // [2] TMA -> MMA
-    uint64_t* x_empty = bars + 2;     // [2] MMA (GEMM 2 done) -> TMA
-    uint64_t* eta_full = bars + 4;    // [2] MMA (GEMM 1 done) -> epilogue
-    uint64_t* eta_empty = bars + 6;   // [2] epilogue (D1 read) -> MMA
-    uint64_t* r_full = bars + 8;      // epilogue (r written) -> MMA
-    uint64_t* r_empty = bars + 9;     // MMA (GEMM 2 done: r and the X stage are free) -> epilogue
-    uint64_t* g_full = bars + 10;     // MMA (drain point reached: D2 holds kTcDrain slabs) -> epilogue
-    uint64_t* g_empty = bars + 11;    // epilogue (D2 drained) -> MMA
-    __shared__ uint32_t tmem_base_s;
-    __shared__ double lp_half_s[kTcChains];
-
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int c_base = blockIdx.y * kTcChains;
-    // slabs of this CTA: blockIdx.x, blockIdx.x + gridDim.x, ...
-    const long long my_slabs = (A.n_slabs > blockIdx.x) ? (A.n_slabs - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
-
-    if (tid == 0) {
-        for (int i = 0; i < 2; ++i) {
-            mbar_init(&x_full[i], 1);
-            mbar_init(&x_empty[i], 1);
-            mbar_init(&eta_full[i], 1);
-            mbar_init(&eta_empty[i], kTcEpiThreads);
-        }
-        mbar_init(r_full, kTcEpiThreads);
-        mbar_init(r_empty, 1);
-        mbar_init(g_full, 1);
-        mbar_init(g_empty, kTcEpiThreads);
-    }
-    if (warp == 1) {  // TMEM: all 512 columns (1 CTA per SM by construction: 193 KB of shared memory)
-        const uint32_t ncols = 512;
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_s)), "r"(ncols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    // beta pieces: fp64 -> fp16 hi / lo, written in the K-major SWIZZLE_128B image GEMM 1 reads as operand A
-    for (int e = tid; e < kTcChains * kTcK; e += kTcThreads) {
-        const int c = e >> 7, k = e & 127;
-        const double v = (c_base + c < A.C && k < A.K) ? A.Q[(long long)(c_base + c) * A.ldq + k] : 0.0;
-        const __half hi = __double2half(v);
-        const __half lo = __double2half(v - (double)__half2float(hi));
-        const uint32_t off = tc_tile_off(c, k);
-        *reinterpret_cast<__half*>(beta_s + off) = hi;
-        *reinterpret_cast<__half*>(beta_s + kTcPieceBytes + off) = lo;
-    }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy writes of beta -> visible to the MMA (async proxy)
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem = tmem_base_s;
-    const uint32_t tD1[2] = {tmem + 0, tmem + 128}, tD2 = tmem + 256, tRh = tmem + 384, tRl = tmem + 448;
-
-    if (warp == 0) {
-        // ===== TMA producer =====
-        if (lane == 0) {
-            for (long long s = 0; s < my_slabs; ++s) {
-                const int st = (int)(s % kTcStages);
-                if (s >= kTcStages) tc_mbar_wait(&x_empty[st], (uint32_t)(((s / kTcStages) - 1) & 1));
-                const long long slab = blockIdx.x + s * gridDim.x;
-                const int row0 = (int)(slab * kTcRows);
-                char* dst = x_s + st * kTcStageBytes;
-                mbar_expect_tx(&x_full[st], kTcStageBytes);
-                tc_tma_load_2d(dst, &map_hi, 0, row0, &x_full[st]);
-                tc_tma_load_2d(dst + kTcBlockBytes, &map_hi, 64, row0, &x_full[st]);
-                tc_tma_load_2d(dst + kTcPieceBytes, &map_lo, 0, row0, &x_full[st]);
-                tc_tma_load_2d(dst + kTcPieceBytes + kTcBlockBytes, &map_lo, 64, row0, &x_full[st]);
-            }
-        }
-    } else if (warp == 1) {
-        // ===== MMA issuer (one lane) =====
-        if (lane == 0) {
-            const uint32_t beta_a = smem_u32(beta_s);
-            auto gemm1 = [&](long long s) {  // D1[s & 1] = beta . X^T   (3 products x 8 k-steps, small products first)
-                const int st = (int)(s % kTcStages), b = (int)(s & 1);
-                tc_mbar_wait(&x_full[st], (uint32_t)((s / kTcStages) & 1));
-                if (s >= 2) tc_mbar_wait(&eta_empty[b], (uint32_t)(((s >> 1) - 1) & 1));
-                tc_fence_after();
-                const uint32_t xa = smem_u32(x_s + st * kTcStageBytes);
-                uint32_t acc = 0;
-#pragma unroll
-                for (int prod = 0; prod < 3; ++prod) {  // hi*lo, lo*hi, hi*hi
-                    const uint32_t a0 = beta_a + (prod == 1 ? kTcPieceBytes : 0);
-                    const uint32_t b0 = xa + (prod == 0 ? kTcPieceBytes : 0);
-#pragma unroll
-                    for (int ks = 0; ks < 8; ++ks) {
-                        const uint32_t o = (uint32_t)((ks >> 2) * kTcBlockBytes + (ks & 3) * 32);
-                        tc_mma_ss(tD1[b], tc_desc(a0 + o, 16, 1024), tc_desc(b0 + o, 16, 1024), kTcIdesc, acc);
-                        acc = 1;
-                    }
-                }
-                tc_commit(&eta_full[b]);
-            };
-            if (my_slabs > 0) gemm1(0);
-            for (long long s = 0; s < my_slabs; ++s) {
-                if (s + 1 < my_slabs) gemm1(s + 1);
-                // GEMM 2 of slab s: D2 = r . X   (A = r pieces in TMEM, B = X pieces read MN-major); D2 was drained
-                tc_mbar_wait(r_full, (uint32_t)(s & 1));
-                const bool first = (s % kTcDrain) == 0;   // D2 was drained before this slab
-                if (first && s > 0) tc_mbar_wait(g_empty, (uint32_t)(((s / kTcDrain) - 1) & 1));
-                tc_fence_after();
-                const int st = (int)(s % kTcStages);
-                const uint32_t xa = smem_u32(x_s + st * kTcStageBytes);
-                uint32_t acc = first ? 0u : 1u;
-#pragma unroll
-                for (int prod = 0; prod < 3; ++prod) {  // r_hi X_lo, r_lo X_hi, r_hi X_hi
-                    const uint32_t ta = (prod == 1) ? tRl : tRh;
-                    const uint32_t b0 = xa + (prod == 0 ? kTcPieceBytes : 0);
-#pragma unroll
-                    for (int ks = 0; ks < 8; ++ks) {  // 16 rows of the slab per step: 2 KB of each 64-column block
-                        tc_mma_ts(tD2, ta + ks * 8, tc_desc(b0 + ks * 2048, kTcBlockBytes, 1024), kTcIdescBmn, acc);
-                        acc = 1;
-                    }
-                }
-                tc_commit(&x_empty[st]);
-                tc_commit(r_empty);
-                if ((s + 1) % kTcDrain == 0 || s + 1 == my_slabs) tc_commit(g_full);
-            }
-        }
-    } else {
-        // ===== epilogue: 8 warps; TMEM lane = chain (subpartition = warp % 4), the two warps of a subpartition split the
-        //       slab's 128 rows (and the 128 gradient columns of a drain) in halves =====
-        const int sub = warp & 3, half = (warp - 2) >> 2;
-        const int c = sub * 32 + lane;                       // chain inside the CTA = TMEM lane
-        const uint32_t lane_addr = (uint32_t)(sub * 32) << 16;
-        double lp = 0.0;
-        // this CTA's fp64 partial gradient, FEATURE-major [128 k][Cpad chains]: for a fixed k the 32 lanes of a warp touch 32
-        // consecutive chains (coalesced read-modify-write in L2; the chain-major layout cost 5 ms per batch, measured)
-        double* gp = A.Gpart + ((long long)blockIdx.x * kTcK + half * 64) * A.Cpad + c_base + c;
-        bool g_first = true;
-        long long n_drains = 0;
-        auto drain = [&]() {  // fp32 gradient accumulator -> fp64 partial
-            tc_mbar_wait(g_full, (uint32_t)(n_drains & 1));
-            tc_fence_after();
-#pragma unroll 1
-            for (int j = 0; j < 2; ++j) {
-                uint32_t v[32];
-                tc_ld32(tD2 + lane_addr + half * 64 + j * 32, v);
-                tc_wait_ld();
-#pragma unroll
-                for (int k = 0; k < 32; ++k) {
-                    const double add = (double)__uint_as_float(v[k]);
-                    double* e = gp + (long long)(j * 32 + k) * A.Cpad;
-                    *e = g_first ? add : *e + add;
-                }
-            }
-            g_first = false;
-            ++n_drains;
-            tc_fence_before();
-            tc_mbar_arrive(g_empty);
-        };
-        for (long long s = 0; s < my_slabs; ++s) {
-            const int b = (int)(s & 1);
-            const long long row0 = (blockIdx.x + s * gridDim.x) * kTcRows + half * 64;
-            tc_mbar_wait(&eta_full[b], (uint32_t)((s >> 1) & 1));
-            tc_fence_after();
-            float lp_s = 0.f;
-            uint32_t rh[2][16], rl[2][16];
-#pragma unroll
-            for (int j = 0; j < 2; ++j) {  // 32 rows of the slab at a time
-                uint32_t v[32];
-                tc_ld32(tD1[b] + lane_addr + half * 64 + j * 32, v);
-                tc_wait_ld();
-                if (j == 1) {  // this thread's share of D1[b] has been read: GEMM 1 of slab s + 2 may overwrite it
-                    tc_fence_before();
-                    tc_mbar_arrive(&eta_empty[b]);
-                }
-                const long long r_base = row0 + j * 32;
-                // y of these 32 rows: one 32-byte global read, the same address for every thread (L1 broadcast)
-                uint32_t yw[8];
-                if (r_base + 32 <= A.N && ((uintptr_t)(A.y + r_base) & 3) == 0) {
-#pragma unroll
-                    for (int w = 0; w < 8; ++w) yw[w] = __ldg(reinterpret_cast<const uint32_t*>(A.y + r_base) + w);
-                } else {
-#pragma unroll
-                    for (int w = 0; w < 8; ++w) {
-                        uint32_t p = 0;
-                        for (int bb = 0; bb < 4; ++bb) {
-                            const long long rr = r_base + 4 * w + bb;
-                            p |= (uint32_t)(rr < A.N ? A.y[rr] : 0) << (8 * bb);
-                        }
-                        yw[w] = p;
-                    }
-                }
-#pragma unroll
-                for (int i = 0; i < 32; i += 2) {
-                    float rr[2];
-#pragma unroll
-                    for (int u = 0; u < 2; ++u) {
-                        const float x = __uint_as_float(v[i + u]);
-                        const float yi = (float)((yw[(i + u) >> 2] >> (8 * ((i + u) & 3))) & 0xff);
-                        const bool live = r_base + i + u < A.N;
-                        const float e = __expf(-fabsf(x));                     // 2 ulp: unbiased, enters sigmoid and log1p only
-                        const float inv = __fdividef(1.f, 1.f + e);
-                        const float sg = x >= 0.f ? inv : e * inv;            // sigmoid(x)
-                        // softplus(x) = max(x, 0) + log(1 + e), 1 + e in (1, 2]: lg2.approx there is good to 2^-22 absolute, four
-                        // times coarser than log1pf but 25 instructions cheaper per element (the epilogue bounds this kernel);
-                        // summed over 1e6 rows that is ~3e-10 of logp, far below the tensor cores' accumulate rounding (1.5e-7)
-                        const float sp = fmaxf(x, 0.f) + __logf(1.f + e);
-                        lp_s += live ? fmaf(yi, x, -sp) : 0.f;
-                        rr[u] = live ? yi - sg : 0.f;
-                    }
-                    const __half2 h = __floats2half2_rn(rr[0], rr[1]);
-                    const float2 hf = __half22float2(h);
-                    const __half2 l = __floats2half2_rn(rr[0] - hf.x, rr[1] - hf.y);
-                    rh[j][i >> 1] = *reinterpret_cast<const uint32_t*>(&h);
-                    rl[j][i >> 1] = *reinterpret_cast<const uint32_t*>(&l);
-                }
-            }
-            // GEMM 2 of the previous slab has finished by now (it ran under the arithmetic above), which frees r for this slab;
-            // every kTcDrain slabs its accumulator goes to fp64
-            if (s > 0) {
-                if (s % kTcDrain == 0) drain();
-                else {
-                    tc_mbar_wait(r_empty, (uint32_t)((s - 1) & 1));
-                    tc_fence_after();
-                }
-            }
-#pragma unroll
-            for (int j = 0; j < 2; ++j) {
-                tc_st16(tRh + lane_addr + half * 32 + j * 16, rh[j]);
-                tc_st16(tRl + lane_addr + half * 32 + j * 16, rl[j]);
-            }
-            tc_wait_st();
-            tc_fence_before();
-            tc_mbar_arrive(r_full);
-            lp += (double)lp_s;
-        }
-        if (my_slabs > 0) drain();
-        else {
-            for (int k = 0; k < 64; ++k) gp[(long long)k * A.Cpad] = 0.0;
-        }
-        if (half == 1) lp_half_s[c] = lp;
-        __syncwarp();
-        asm volatile("bar.sync 1, %0;" ::"r"(kTcEpiThreads) : "memory");  // the 8 epilogue warps only
-        if (half == 0) A.lpart[(long long)blockIdx.x * A.Cpad + c_base + c] = lp + lp_half_s[c];
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) {
-        tc_fence_after();
-        const uint32_t ncols = 512;
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(ncols) : "memory");
-    }
-}
-
-// =========================================================================================================================
-// Version 2 of the kernel above (round 2, second session).  Same GEMMs, same TMEM map, same accumulate order and drain period;
-// what changed is everything around them, after the ncu capture of version 1 (profiles/r2_tc_logistic_tc_ncu_summary.csv:
-// tensor pipe 14 % busy, 63 warp-instructions per (row, chain) element, 42 % of the stall samples on long-scoreboard waits):
-//   * 16 epilogue warps instead of 8 (four per TMEM subpartition, 32 rows of the slab each): 4 warps per scheduler hide the
-//     TMEM-load and MUFU latencies that 2 could not;
-//   * the gradient partials stay in REGISTERS as fp64 (32 per thread) across the drains and are written once at the end:
-//     version 1 added every drain into global memory (2 x 64 read-modify-writes per thread every 2 slabs = 2 GB of L2
-//     traffic per launch, the long-scoreboard stalls);
-//   * y travels with the slab: the TMA producer copies the slab's 128 labels (fp32, 512 B) into the stage next to the X pieces
-//     (version 1 read them from global memory inside the element loop and converted bytes to floats per element);
-//   * elementwise math on the MUFU units directly (ex2 / rcp / lg2 .approx.ftz): 12 instructions per element for
-//     sigmoid + softplus + log-likelihood + residual; fp16 pieces of the residual are packed in place;
-//   * rows past N need no masking: their X rows are zero, so eta = 0 exactly, the residual multiplies zero rows in GEMM 2, and
-//     the log-likelihood they add (-softplus(0) each) is added back per slab.
 constexpr int kTc2EpiWarps = 16;
 constexpr int kTc2EpiThreads = 32 * kTc2EpiWarps;
 constexpr int kTc2Threads = 64 + kTc2EpiThreads;  // TMA producer, MMA issuer, 16 epilogue warps
 constexpr uint32_t kTc2YBytes = kTcRows * sizeof(float);
-constexpr size_t kTc2SmemBytes = kTcSmemBytes + kTcStages * kTc2YBytes;
+constexpr size_t kTc2SmemBytes = 1024 /*align*/ + 2 * kTcPieceBytes /*beta hi, lo*/ + kTcStages * kTcStageBytes + 256 /*barriers*/ +
+                                 kTcStages * kTc2YBytes /*labels*/;
 
 __device__ __forceinline__ float tc_ex2(float x) { float r; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x)); return r; }
 __device__ __forceinline__ float tc_rcp(float x) { float r; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x)); return r; }
@@ -530,7 +244,7 @@ __global__ void __launch_bounds__(kTc2Threads, 1)
             }
         }
     } else if (warp == 1) {
-        // ===== MMA issuer (one lane): identical to version 1 =====
+        // ===== MMA issuer (one lane) =====
         if (lane == 0) {
             const uint32_t beta_a = smem_u32(beta_s);
             auto gemm1 = [&](long long s) {
@@ -703,7 +417,7 @@ __global__ void __launch_bounds__(kTc2Threads, 1)
     }
 }
 
-// labels as fp32, zero padded to whole slabs (version 2 copies them into shared memory with the slab)
+// labels as fp32, zero padded to whole slabs (logistic_tc2_kernel copies them into shared memory with the slab)
 __global__ void __launch_bounds__(256) logistic_tc_y_kernel(const uint8_t* __restrict__ y, long long N, float* __restrict__ y32,
                                                             long long rows_pad) {
     const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;

@@ -10,10 +10,6 @@
 #pragma once
 #include "common.cuh"
 
-#ifndef B200_EVAL_INLINE
-#define B200_EVAL_INLINE  // define as __noinline__ to keep one copy of the model function (I-cache footprint)
-#endif
-
 namespace b200 {
 
 // ------------------------------------------------------------------------------------------------
@@ -125,7 +121,7 @@ struct RadonModel {
     }
 
     template <int NPL, int W, bool SMALL = false>
-    __device__ B200_EVAL_INLINE static double eval(const Params& P, const char* smem, const double* q_s, double* g_s, int lane,
+    __device__ static double eval(const Params& P, const char* smem, const double* q_s, double* g_s, int lane,
                                                    double*) {
         static_assert(W == 1, "RadonModel is a chain-per-warp model");
         const double2* xy = reinterpret_cast<const double2*>(smem) + lane;

@@ -99,28 +99,21 @@ __host__ __device__ inline long long nuts_scratch_doubles(int NP, int levels) {
     return (long long)(G_STACK + 4 * levels) * NP;
 }
 // shared memory per warp (bytes): q, g, hot stack levels (level 0: 2 vectors, others: 4), scalars
-#ifndef B200_SUBTREE_SMEM
-#define B200_SUBTREE_SMEM 0  // 1: left.p / p_sum / proposal q of the subtree under construction live in shared memory
-#endif                       //    (frees 6*NPL registers per lane -> more resident warps); 0: in registers
 // (per chain; + 3 vectors when the subtree under construction is kept in shared memory; + the team's reduction pad)
-__host__ __device__ inline size_t nuts_warp_smem_bytes(int NP, int hot, bool subs = B200_SUBTREE_SMEM, int W = 1) {
+__host__ __device__ inline size_t nuts_warp_smem_bytes(int NP, int hot, bool subs, int W) {
     const int vecs = 2 + (subs ? 3 : 0) + (hot > 0 ? 2 + 4 * (hot - 1) : 0);
     return (size_t)vecs * NP * sizeof(double) + 5 * kMaxLevels * sizeof(double) +
            (W > 1 ? W * 8 * sizeof(double) : 0);
 }
 
-#ifndef B200_NUTS_THREADS
-#define B200_NUTS_THREADS 256  // CTA size cap of the NUTS kernel (warps per CTA <= THREADS/32)
-#endif
-#ifndef B200_NUTS_MINBLOCKS
-#define B200_NUTS_MINBLOCKS 1  // __launch_bounds__ min CTAs/SM: the register budget knob
-#endif
-// W = warps per chain (team).  SUBS = subtree-under-construction vectors in shared memory instead of registers.
+// chains (warps) per CTA of the chain-per-warp kernel: 8 warps, 1 CTA per SM (measured best, round 2)
+constexpr int kNutsWarpChains = 8;
+// W = warps per chain (team).  SUBS: left.p / p_sum / proposal q of the subtree under construction live in shared memory
+// (a team, W > 1) or in registers (a warp, W = 1).
 // Register caps below the ~240 the kernel wants were measured and rejected (round 2, profiles/r2_variants.md): 224 registers
 // (9 warps/SM) 460 ms, 200 (10 warps/SM, 264 B of spills) 521 ms, 168 (12 warps/SM) 685 ms vs 370 ms at 2 x 4 warps per SM.
-#define B200_NUTS_BOUNDS __launch_bounds__(W > 1 ? 32 * W : B200_NUTS_THREADS, W > 1 ? 1 : B200_NUTS_MINBLOCKS)
-template <class Model, int NPL, int W, bool SUBS>
-__global__ void B200_NUTS_BOUNDS
+template <class Model, int NPL, int W, bool SUBS = (W > 1)>
+__global__ void __launch_bounds__(W > 1 ? 32 * W : 32 * kNutsWarpChains, 1)
     nuts_warp_kernel(const NutsDev P, const typename Model::Params M) {
     constexpr int TS = 32 * W;      // threads per chain
     constexpr int NP = TS * NPL;    // padded vector length

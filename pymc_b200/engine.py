@@ -117,9 +117,8 @@ class CompiledModel:
                 kind[sl] = 1
             elif v.transform == "interval":
                 kind[sl], lo[sl], hi[sl] = 2, v.bounds[0], v.bounds[1]
-        self.supports_constrain = hasattr(self._lib, "b200_model_set_transforms")
-        if self.supports_constrain:
-            _lib.check(self._lib.b200_model_set_transforms(self._h, kind.ctypes.data, lo.ctypes.data, hi.ctypes.data))
+        self.supports_constrain = True
+        _lib.check(self._lib.b200_model_set_transforms(self._h, kind.ctypes.data, lo.ctypes.data, hi.ctypes.data))
 
     def pointwise_loglik(self, draws, lik: int = 0):
         """log p(y_i | draw) for every draw: ``draws[..., n]`` (unconstrained) -> ``[..., N]`` (IR models on the generic

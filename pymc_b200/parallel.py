@@ -202,8 +202,6 @@ class near_gpu:
     def __enter__(self):
         import os
 
-        if os.environ.get("B200_NO_NUMA_BIND"):
-            return self
         node, cpus = gpu_numa_cpus(self.device)
         self.info["numa_node"] = node
         try:

@@ -25,10 +25,9 @@ if [ "$PART" = bench ]; then
   echo "launch list rc=$?"
 elif [ "$PART" = tc ]; then
   timeout -k 10 200 $NCU --metrics gpu__time_duration.sum -c 300 --csv --log-file $O/${R}_launches_logistic_tc.csv python scripts/ncu_target3.py logistic_tc 4 2 > $O/${R}_launches_logistic_tc.log 2>&1
-  cap logistic_tc logistic_tc_kernel 2 scripts/ncu_target3.py logistic_tc 2 1
   timeout -k 10 200 $NCU --metrics gpu__time_duration.sum -c 300 --csv --log-file $O/${R}_launches_mvgauss_tc.csv python scripts/ncu_target3.py mvgauss_tc 4 2 > $O/${R}_launches_mvgauss_tc.log 2>&1
   cap gemm_tc gemm_tc_kernel 4 scripts/ncu_target3.py mvgauss_tc 2 1
-elif [ "$PART" = tc2 ]; then  # version 2 of the tensor-core logistic pass only
+elif [ "$PART" = tc2 ]; then  # the tensor-core logistic pass only
   timeout -k 10 200 $NCU --metrics gpu__time_duration.sum -c 300 --csv --log-file $O/${R}_launches_logistic_tc.csv python scripts/ncu_target3.py logistic_tc 4 2 > $O/${R}_launches_logistic_tc.log 2>&1
   cap logistic_tc logistic_tc2_kernel 2 scripts/ncu_target3.py logistic_tc 2 1
 elif [ "$PART" = stochvol ]; then

@@ -27,7 +27,7 @@ for (name, c), dn in zip(kern.items(), demangle):
     short = re.sub(r"\(.*", "", dn).replace("void ", "").replace("b200::", "")
     rows.append((short, c))
 want = sys.argv[1:] or ["nuts_warp_kernel<RadonModel, 6", "nuts_warp_kernel<StochVolModel, 12", "nuts_warp_kernel<IrModel, 6, 1", "logistic_fused_kernel<16",
-                        "gemm_nt_dmma_kernel<8, 17", "logistic_tc_kernel", "gemm_tc_kernel", "ls_advance_kernel<16", "ls_advance_kernel<1",
+                        "gemm_nt_dmma_kernel<8, 17", "gemm_tc_kernel", "ls_advance_kernel<16", "ls_advance_kernel<1",
                         "logp_grad_warp_kernel<RadonModel, 6", "ir_pointwise_kernel"]
 with open(os.path.join(ROOT, "profiles", "r2_sass_opcodes.md"), "w") as f:
     f.write(f"# SASS opcode counts per kernel (static, `cuobjdump -sass pymc_b200/libb200nuts.so`), built from commit `{commit}` + working tree\n\n")

@@ -227,9 +227,8 @@ def test_lockstep_row_compaction_changes_nothing(case, monkeypatch):
         A = np.random.default_rng(0).standard_normal((spec.n, spec.n)) * 0.05
         cm.set_dense_mass(cov=np.eye(spec.n) * 0.05 + A @ A.T)
         kw = dict(tune=20, draws=6, mass="dense")
-    monkeypatch.setenv("B200_LS_COMPACT", "0")
+    monkeypatch.setenv("B200_LS_COMPACT_TILE", "0")
     ref = _lockstep_run(cm, 40, **kw)
-    monkeypatch.setenv("B200_LS_COMPACT", "1")
     monkeypatch.setenv("B200_LS_COMPACT_TILE", "8")
     got = _lockstep_run(cm, 40, **kw)
     ge = ref.summary["grad_evals"]
